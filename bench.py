@@ -232,8 +232,34 @@ def _drive_reference(args, ray_train) -> dict:
             "dtype": "fp32 (thinc default)", "data": "synthetic (same generator, written as DocBin)"}
 
 
-def run_arm(args, impl: str, rank: int, world: int, local_rank: int):
-    """One measured arm (``ours`` / ``nccl-baseline``).  Returns the result dict on every rank."""
+DUMP_BYTES = 64 << 20
+
+
+def dump_outputs(out_dir: str, losses, proxy) -> None:
+    """Write what the last timed step hands its caller: ``losses.npy`` (per-head losses, ``loss_names`` order)
+    and ``params.npy`` (every parameter after the optimizer update, layout order, padding left out), both
+    float32.  Parameters beyond the byte budget are replaced by a fixed, seeded sample of them.  The inputs are
+    seeded, but some device sums accumulate in a varying order: two runs agree to rounding after a few steps and
+    drift apart over hundreds, so compare two builds at a small ``--steps``."""
+    import numpy as np
+    import torch
+
+    lay = proxy.layout
+    idx = torch.cat([torch.arange(lay.offset[k], lay.offset[k] + lay.numel[k]) for k in lay.keys])
+    cap = (DUMP_BYTES - 4 * losses.numel()) // 4
+    if idx.numel() > cap:
+        pick = np.sort(np.random.default_rng(0).choice(idx.numel(), size=cap, replace=False))
+        idx = idx[torch.from_numpy(pick)]
+    params = proxy.param_flat[idx.to(proxy.param_flat.device)].float().cpu().numpy()
+    out = Path(out_dir)
+    out.mkdir(parents=True, exist_ok=True)
+    np.save(out / "losses.npy", losses.detach().float().cpu().numpy())
+    np.save(out / "params.npy", params)
+
+
+def run_arm(args, impl: str, rank: int, world: int, local_rank: int, steps: int, dump_dir=None):
+    """One measured arm (``ours`` / ``nccl-baseline``) of ``steps`` timed steps.  Returns the result dict on
+    every rank.  With ``dump_dir``, rank 0 writes the outputs of the last timed step there (``dump_outputs``)."""
     import numpy as np
     import torch
     import torch.distributed as dist
@@ -294,9 +320,7 @@ def run_arm(args, impl: str, rank: int, world: int, local_rank: int):
     use_graphs = args.engine == "graph" and impl == "ours"
     trainer = Trainer(nlp, proxy, examples, docs_per_batch=B, dropout=args.dropout, use_graphs=use_graphs,
                       bucket_rows=args.bucket_rows)
-    steps, warmup = args.steps, args.warmup
-    if impl != "ours":
-        steps = min(steps, args.baseline_steps)
+    warmup = args.warmup
     n_total = warmup + steps
     # token-balanced batches: every rank's every batch holds exactly B * (min_len + max_len) / 2 tokens,
     # so all ranks run the same row count each step (a synchronous step is as slow as its largest batch)
@@ -332,9 +356,11 @@ def run_arm(args, impl: str, rank: int, world: int, local_rank: int):
         barrier()
         evs[0].record()
         for i, item in enumerate(dev_inputs[warmup: n_total]):
-            device_step(item)
+            losses = device_step(item)
             evs[i + 1].record()
         barrier()
+    if dump_dir is not None and rank == 0:
+        dump_outputs(dump_dir, losses, proxy)
     ms = max_over_ranks(float(evs[0].elapsed_time(evs[-1])))
     per_step = sorted(float(evs[i].elapsed_time(evs[i + 1])) for i in range(steps))
     launches = ops.launches + getattr(proxy.comm, "launches", 0) - launches0
@@ -452,7 +478,12 @@ def main() -> int:
     ap.add_argument("--no-own-baseline", dest="own_baseline", action="store_false",
                     help="skip the nccl-baseline arm that is otherwise run after the product arm")
     ap.add_argument("--baseline-steps", type=int, default=20)
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps, write the losses and updated parameters of the last one to "
+                         "DIR/*.npy (float32, at most 64 MB) so that two builds can be compared on identical inputs")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
 
     if args.impl == "reference":
         return reference_arm(args)
@@ -479,13 +510,13 @@ def main() -> int:
         print(json.dumps({"impl": args.impl, "unavailable": "rayproxy-emu runs under the actor runtime: "
                           "use benchmarks/bench_rayproxy.py"}))
         return 0
-    out = run_arm(args, args.impl, rank, world, local_rank)
+    out = run_arm(args, args.impl, rank, world, local_rank, args.steps, dump_dir=args.dump_outputs)
     if args.impl == "ours" and args.own_baseline:
         # OUR emulation of an NCCL(+cuBLAS) build of the reference's data flow, same box, same N, same
         # metric/config - context for the reader; the published-number ratio `vs_baseline` stays null
         # because the reference publishes nothing (BASELINE.md)
         try:
-            base = run_arm(args, "nccl-baseline", rank, world, local_rank)
+            base = run_arm(args, "nccl-baseline", rank, world, local_rank, min(args.steps, args.baseline_steps))
             out["vs_own_nccl_baseline"] = {
                 "ratio": out["value"] / base["value"], "baseline_value": base["value"], "baseline_steps": base["steps"],
                 "baseline_ms_per_step": base["ms_per_step"],

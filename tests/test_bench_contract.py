@@ -1,10 +1,13 @@
-"""The parts of ``bench.py``'s driver contract that can be checked without a GPU: the reference arm really
-tries to import the reference and reports the exception text; the argument surface the driver uses exists;
-the flagship config is the model BASELINE.json names."""
+"""``bench.py``'s command-line contract.  Without a GPU: the reference arm really tries to import the reference
+and reports the exception text; the documented flags exist; the flagship config is the model BASELINE.json
+names.  On a GPU: ``--steps`` is the number of timed steps and ``--dump-outputs`` writes the last step's outputs."""
 import json
 import subprocess
 import sys
 from pathlib import Path
+
+import numpy as np
+import pytest
 
 ROOT = Path(__file__).resolve().parent.parent
 
@@ -29,7 +32,7 @@ def test_reference_arm_prints_one_json_line_with_the_real_reason():
 def test_cli_surface_the_driver_uses():
     out = _run("--help")
     assert out.returncode == 0
-    for flag in ("--gpus", "--steps", "--warmup", "--impl", "--config", "--no-own-baseline"):
+    for flag in ("--gpus", "--steps", "--warmup", "--impl", "--config", "--no-own-baseline", "--dump-outputs"):
         assert flag in out.stdout, flag
 
 
@@ -49,3 +52,30 @@ def test_flagship_config_is_the_named_model():
     assert t2v["encode"]["width"] == 256 and t2v["encode"]["depth"] == 8 and t2v["encode"]["maxout_pieces"] == 3
     base = json.loads((ROOT / "BASELINE.json").read_text())
     assert "tok2vec+NER" in base["metric"]
+
+
+def test_zero_steps_is_rejected():
+    out = _run("--steps", "0")
+    assert out.returncode != 0 and "--steps" in out.stderr
+
+
+@pytest.mark.gpu
+@pytest.mark.parametrize("impl", ["ours", "nccl-baseline"])
+def test_steps_are_timed_and_last_step_outputs_dumped(tmp_path, impl):
+    small = ("--docs-per-gpu", "64", "--no-e2e", "--no-own-baseline", "--baseline-steps", "2")
+    dumps = []
+    for run in ("a", "b"):
+        out = _run("--impl", impl, "--gpus", "1", "--steps", "3", "--warmup", "3", *small,
+                   "--dump-outputs", str(tmp_path / run))
+        assert out.returncode == 0, out.stderr[-2000:]
+        line = json.loads(out.stdout.strip().splitlines()[-1])
+        assert line["impl"] == impl and line["steps"] == 3       # --baseline-steps caps only the context arm
+        dumps.append({f.name: np.load(f) for f in sorted((tmp_path / run).iterdir())})
+    a, b = dumps
+    assert set(a) == {"losses.npy", "params.npy"} and sum(x.nbytes for x in a.values()) <= 64 << 20
+    assert a["losses.npy"].dtype == np.float32 and a["params.npy"].dtype == np.float32
+    assert a["losses.npy"].shape == (1,) and np.isfinite(a["losses.npy"]).all() and a["losses.npy"][0] > 0
+    assert a["params.npy"].shape == b["params.npy"].shape and np.isfinite(a["params.npy"]).all()
+    # same arguments, same inputs: two runs agree up to the order of floating-point accumulation
+    assert np.allclose(a["losses.npy"], b["losses.npy"], rtol=1e-2)
+    assert np.abs(a["params.npy"] - b["params.npy"]).max() < 1e-2
