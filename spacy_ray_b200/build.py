@@ -28,7 +28,7 @@ OUT_HOST = ROOT / "native" / "_host_runtime.so"
 OBJ_DIR = ROOT / "ops" / "_build"
 
 NVCC_ARCH = ["-gencode", "arch=compute_100a,code=sm_100a"]
-CU_FILES = ["elementwise_kernels.cu", "elementwise_fast.cu", "ner_kernels.cu", "tagger_kernels.cu", "parser_kernels.cu", "gemm_tcgen05.cu", "comm_kernels.cu"]
+CU_FILES = ["elementwise_kernels.cu", "elementwise_fast.cu", "ner_kernels.cu", "tagger_kernels.cu", "parser_kernels.cu", "gemm_tcgen05.cu", "comm_kernels.cu", "textcat_kernels.cu"]
 CPP_FILES = ["bindings.cpp", "gemm_binding.cpp", "comm_binding.cpp"]
 
 

@@ -18,10 +18,10 @@ issues a few hundred small launches per step from Python; on a B200 that is
 * **one 4-byte D2H read** of the loss.
 
 Supports any pipeline made of the built-in trainable components - a shared
-``tok2vec`` plus ``tagger`` / ``ner`` / ``parser`` heads, each with its own or a listener
-tok2vec (the whole of SURVEY.md 2.6's component list) - as long as the transition heads fit
-their device kernels (``Trainer.unsupported_reason``).  Everything else uses the generic
-``nlp.update`` path.
+``tok2vec`` plus ``tagger`` / ``ner`` / ``parser`` / ``textcat`` heads, each with its own or a
+listener tok2vec (the whole of SURVEY.md 2.6's component list) - as long as the transition and
+textcat heads fit their device kernels (``Trainer.unsupported_reason``).  Everything else uses the
+generic ``nlp.update`` path.
 """
 from __future__ import annotations
 
@@ -49,11 +49,13 @@ def _align(x: int, a: int = 256) -> int:
 def _kind(comp) -> Optional[str]:
     """Which device-side step serves a component.  Every token tagger (``Tagger`` and its subclasses
     ``SentenceRecognizer`` / ``Morphologizer``: same model, same kernels, only the gold ids differ) is a
-    "tagger"."""
-    from ..pipeline.components import Tagger
+    "tagger"; both document classifiers are a "textcat"."""
+    from ..pipeline.components import Tagger, TextCategorizer
 
     if isinstance(comp, Tagger):
         return "tagger"
+    if isinstance(comp, TextCategorizer):          # textcat and textcat_multilabel
+        return "textcat"
     return {"Tok2VecComponent": "tok2vec", "EntityRecognizer": "ner",
             "DependencyParser": "parser"}.get(comp.__class__.__name__)
 
@@ -62,7 +64,9 @@ class ExampleStore:
     """Structure-of-arrays view of a list of Examples: attribute ids plus one int32 gold
     array per head.  ``slots[key] = (array, doc_off, padded)``: token-order arrays share
     ``doc_off``; *padded* arrays carry one trailing ``-1`` per doc so that a plain per-doc
-    memcpy lands them in the padded-ragged row layout (the tagger's labels)."""
+    memcpy lands them in the padded-ragged row layout (the tagger's labels).  ``cats[key] = (truths,
+    known)``: per-document (n_docs, n_labels) fp32 arrays of a textcat head, exactly what
+    ``TextCategorizer._truths`` builds (a label missing from ``Doc.cats`` is "unknown")."""
 
     def __init__(self, examples: Sequence[Any], heads: Sequence[tuple]) -> None:
         lens = np.array([len(eg) for eg in examples], dtype=np.int64)
@@ -81,6 +85,7 @@ class ExampleStore:
             self.gid[:, c] = inv.reshape(-1)
             self.n_groups[c] = len(uniq)
         self.slots: Dict[str, tuple] = {}
+        self.cats: Dict[str, tuple] = {}
 
         def cat(parts):
             return np.ascontiguousarray(np.concatenate(parts).astype(np.int32))
@@ -99,6 +104,9 @@ class ExampleStore:
                     parts.append(comp.gold_ids(eg.reference).astype(np.int32))
                     parts.append(end)
                 self.slots[name] = (cat(parts), self.doc_off_padded, True)
+            elif kind == "textcat":
+                truths, known = comp._truths(examples, "cpu")
+                self.cats[name] = (np.ascontiguousarray(truths.numpy()), np.ascontiguousarray(known.numpy()))
         self.lens = lens
         self.n_docs = len(examples)
         self.max_len = int(lens.max()) if len(lens) else 1
@@ -110,6 +118,7 @@ class _Layout:
     docs: int
     lmax: int
     slots: tuple = ()
+    cats: tuple = ()                 # ((textcat head, n_labels), ...)
     bucket: int = 1024
     n_attr: int = 4
     off_attrs: int = 0
@@ -132,6 +141,10 @@ class _Layout:
         self.off_gold = {}
         for key in self.slots:
             self.off_gold[key] = o; o = _align(o + self.rows * 4)
+        self.off_cats = {}
+        for key, n_labels in self.cats:
+            off_t = o; o = _align(o + self.docs * n_labels * 4)
+            self.off_cats[key] = (off_t, o, n_labels); o = _align(o + self.docs * n_labels * 4)
         self.off_scratch = o; o = _align(o + self.docs * 4)
         self.off_perm = o; o = _align(o + self.n_attr * self.rows * 4)
         self.off_inv = o; o = _align(o + self.lmax * 4)
@@ -154,6 +167,8 @@ class _Views:
         self.lens = v(lay.off_lens, lay.docs, torch.int32)
         self.tok_off = v(lay.off_tok, lay.docs, torch.int32)
         self.gold = {k: v(off, lay.rows, torch.int32) for k, off in lay.off_gold.items()}
+        self.cats = {k: tuple(v(off, lay.docs * n, torch.float32).view(lay.docs, n) for off in (ot, ok))
+                     for k, (ot, ok, n) in lay.off_cats.items()}     # textcat (truths, known)
         self.scratch = v(lay.off_scratch, lay.docs, torch.int32)
         self.perm = v(lay.off_perm, lay.n_attr * lay.rows, torch.int32)
         self.inv_active = v(lay.off_inv, lay.lmax, torch.float32)
@@ -167,6 +182,7 @@ def make_stage(lay: _Layout, store: ExampleStore, pin: bool = True) -> dict:
     arrs = {k: getattr(hv, k).numpy() for k in
             ("attrs", "mask", "starts", "lens", "tok_off", "inv_active", "meta", "scratch", "perm")}
     arrs["gold"] = {k: t.numpy() for k, t in hv.gold.items()}
+    arrs["cats"] = {k: (t.numpy(), kn.numpy()) for k, (t, kn) in hv.cats.items()}
     arrs["hist"] = np.zeros(int(store.n_groups.sum()) + len(store.n_groups), dtype=np.int32)
     for key, (_arr, _off, padded) in store.slots.items():
         if padded:
@@ -193,6 +209,13 @@ def fill_stage(st: ExampleStore, lay: _Layout, stage: dict, ids: np.ndarray, his
         else:
             native.collate_gold(arr, doc_off, ids, out, a["tok_off"] if first else a["scratch"])
             first = False
+    n = len(ids)
+    for key, (truths, known) in st.cats.items():   # per-doc textcat truths: one vectorised gather
+        out_t, out_k = a["cats"][key]
+        np.take(truths, ids, axis=0, out=out_t[:n])
+        np.take(known, ids, axis=0, out=out_k[:n])
+        out_t[n:] = 0.0
+        out_k[n:] = 0.0                            # unused doc slots: nothing known
     if first:                                      # no token-order slot filled tok_off
         lens_i = st.lens[ids]
         a["tok_off"][: len(ids)] = (np.cumsum(lens_i) - lens_i).astype(np.int32)
@@ -204,6 +227,7 @@ def fill_stage(st: ExampleStore, lay: _Layout, stage: dict, ids: np.ndarray, his
     counts = (lens[None, :] > np.arange(lay.lmax, dtype=np.int32)[:, None]).sum(axis=1)
     a["inv_active"][:] = 1.0 / np.maximum(counts, 1)
     a["meta"][0] = rows
+    a["meta"][1] = len(ids)                        # real doc count (textcat: loss and gradient scale)
     # HashEmbed backward: rows grouped by id per attribute column, laid out for the row bucket
     # the step will run with (the captured graph reads perm as (n_attr, rb))
     rb = min(lay.rows, _align(int(rows), lay.bucket))
@@ -235,8 +259,36 @@ class Trainer:
                     cap = Trainer.parser_doc_capacity(comp)
                     if max_len > cap:
                         return f"{name}: documents longer than {cap} tokens"
+            if kind == "textcat":
+                why = Trainer.textcat_reason(comp)
+                if why is not None:
+                    return f"{name}: {why}"
         if all(kind == "tok2vec" for _, _, kind in heads):
             return "no head component"
+        return None
+
+    @staticmethod
+    def textcat_reason(comp) -> Optional[str]:
+        """Why the textcat kernels cannot serve this head (None = they can): label count, pooled width
+        (n_pool * width) and n-gram size must fit what one CTA per document holds."""
+        from ..ops.b200_ops import TEXTCAT_MAX_LABELS, TEXTCAT_MAX_NGRAM, TEXTCAT_MAX_POOL
+
+        model = comp.model
+        if "update_with_cats" not in model.attrs:
+            return f"model {model.name!r} has no device-side update"
+        n_labels = len(comp.labels) or model.maybe_get_dim("nO") or 0
+        if n_labels > TEXTCAT_MAX_LABELS:
+            return f"{n_labels} labels (the textcat kernels hold at most {TEXTCAT_MAX_LABELS})"
+        if model.has_ref("output"):
+            pool = model.get_ref("output").maybe_get_dim("nI") or 0
+            if pool > TEXTCAT_MAX_POOL:
+                return f"pooled width {pool} (n_pool * width; the textcat kernels hold at most {TEXTCAT_MAX_POOL})"
+        bow = model.get_ref("linear_model") if model.has_ref("linear_model") else (
+            model if model.name == "textcat_bow" else None)
+        if bow is not None:
+            n = int(bow.attrs.get("ngram_size", 1))
+            if not 1 <= n <= TEXTCAT_MAX_NGRAM:
+                return f"ngram_size {n} (the textcat kernels hash 1 to {TEXTCAT_MAX_NGRAM})"
         return None
 
     @staticmethod
@@ -279,6 +331,7 @@ class Trainer:
         rows_cap = _align(self.B * cap_len + self.B + 1, self.bucket_rows)
         self.lay = _Layout(rows=rows_cap, docs=self.B, lmax=_align(cap_len, 64),
                            slots=tuple(self.store.slots), bucket=self.bucket_rows,
+                           cats=tuple((k, int(t.shape[1])) for k, (t, _kn) in self.store.cats.items()),
                            n_attr=int(self.store.attrs.shape[1]))
         if hasattr(self.ops, "max_rows_hint"):
             self.ops.max_rows_hint = max(int(self.ops.max_rows_hint), int(rows_cap))
@@ -466,6 +519,9 @@ class Trainer:
                 set_dropout_rate(comp.model, self.dropout)
                 if kind == "tagger":
                     loss, _ = comp.model.attrs["update_with_labels"](tb, gold[name][:rows].to(torch.int64))
+                elif kind == "textcat":
+                    truths, known = self.dv.cats[name]
+                    loss, _ = comp.model.attrs["update_with_cats"](tb, truths, known, self.dv.meta[1:2])
                 elif kind == "ner":
                     g = TransitionGold(actions=gold[name][:rows], offsets=None)
                     loss = comp.model.attrs["run"](tb, comp.system, g, True).loss

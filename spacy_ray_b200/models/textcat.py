@@ -81,9 +81,25 @@ def build_textcat_model(tok2vec: Model, exclusive_classes: bool = True, nO: Opti
 
         return scores, backprop
 
+    def update_with_cats(batch: TokenBatch, truths: torch.Tensor, known: torch.Tensor, n_docs):
+        """Forward + loss + backward in one call (``ops.textcat_head``; works on device-resident batches
+        without host lengths).  ``truths`` / ``known``: (B, nO) fp32; ``n_docs``: real doc count (int or
+        a device int32 tensor).  Returns ``(loss, scores)``."""
+        X, bp_t2v = tok2vec(batch, True)
+        W, b = output.get_param("W"), output.get_param("b")
+        go = {"W": output.grad_buffer("W"), "b": output.grad_buffer("b")} if getattr(model.ops, "fused", False) else None
+        loss, scores, dX, grads = model.ops.textcat_head(
+            X, batch, W, b, None, None, truths, known, n_docs=n_docs, use_mean=use_reduce_mean,
+            use_max=use_reduce_max, exclusive=exclusive_classes, grad_out=go)
+        output.inc_grad("W", grads["W"])
+        output.inc_grad("b", grads["b"])
+        bp_t2v(dX)
+        return loss, scores
+
     model = Model("textcat", forward, init=init, dims={"nO": nO},
                   layers=[tok2vec, output], refs={"tok2vec": tok2vec, "output": output})
     model.attrs["exclusive_classes"] = bool(exclusive_classes)
+    model.attrs["update_with_cats"] = update_with_cats
     return model
 
 
@@ -144,10 +160,22 @@ def build_textcat_bow(exclusive_classes: bool = True, ngram_size: int = 1, no_ou
 
         return scores, backprop
 
+    def update_with_cats(batch: TokenBatch, truths: torch.Tensor, known: torch.Tensor, n_docs):
+        """Forward + loss + backward in one call (``ops.textcat_head``); see ``build_textcat_model``."""
+        W, b = model.get_param("W"), model.get_param("b")
+        go = {"W_bow": model.grad_buffer("W"), "b_bow": model.grad_buffer("b")} if getattr(model.ops, "fused", False) else None
+        loss, scores, _dX, grads = model.ops.textcat_head(
+            None, batch, None, None, W, b, truths, known, n_docs=n_docs, use_mean=False, use_max=False,
+            exclusive=exclusive_classes, no_output_layer=no_output_layer, ngram_size=ngram_size, grad_out=go)
+        model.inc_grad("W", grads["W_bow"])
+        model.inc_grad("b", grads["b_bow"])
+        return loss, scores
+
     model = Model("textcat_bow", forward, init=init, dims={"nO": nO}, params={"W": None, "b": None})
     model.attrs["exclusive_classes"] = bool(exclusive_classes)
     model.attrs["no_output_layer"] = bool(no_output_layer)
     model.attrs["ngram_size"] = int(ngram_size)
+    model.attrs["update_with_cats"] = update_with_cats
     return model
 
 
@@ -193,7 +221,29 @@ def build_textcat_ensemble(tok2vec: Model, linear_model: Model, nO: Optional[int
 
         return scores, backprop
 
+    def update_with_cats(batch: TokenBatch, truths: torch.Tensor, known: torch.Tensor, n_docs):
+        """Forward + loss + backward in one call (``ops.textcat_head``); see ``build_textcat_model``.
+        Gradients are handed over in the order the generic backward completes them: the bag of words,
+        the output layer, then the tok2vec."""
+        X, bp_t2v = t2v(batch, True)
+        W, b = neural_out.get_param("W"), neural_out.get_param("b")
+        Wb, bb = linear_model.get_param("W"), linear_model.get_param("b")
+        go = None
+        if getattr(model.ops, "fused", False):
+            go = {"W": neural_out.grad_buffer("W"), "b": neural_out.grad_buffer("b"),
+                  "W_bow": linear_model.grad_buffer("W"), "b_bow": linear_model.grad_buffer("b")}
+        loss, scores, dX, grads = model.ops.textcat_head(
+            X, batch, W, b, Wb, bb, truths, known, n_docs=n_docs, use_mean=True, use_max=False, exclusive=exclusive,
+            ngram_size=int(linear_model.attrs.get("ngram_size", 1)), grad_out=go)
+        linear_model.inc_grad("W", grads["W_bow"])
+        linear_model.inc_grad("b", grads["b_bow"])
+        neural_out.inc_grad("W", grads["W"])
+        neural_out.inc_grad("b", grads["b"])
+        bp_t2v(dX)
+        return loss, scores
+
     model = Model("textcat_ensemble", forward, init=init, dims={"nO": nO},
                   layers=[neural, linear_model], refs={"tok2vec": t2v, "output": neural_out, "linear_model": linear_model})
     model.attrs["exclusive_classes"] = exclusive
+    model.attrs["update_with_cats"] = update_with_cats
     return model

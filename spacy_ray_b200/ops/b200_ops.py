@@ -43,6 +43,8 @@ _LIB = Path(__file__).parent / "_srb_cuda.so"
 _loaded = False
 
 MODE_KK, MODE_MNMN, MODE_KMN = 0, 1, 2
+# what the textcat kernels hold (csrc/kernels.h kTextcat*): labels, n_pool * width, ngram_size
+TEXTCAT_MAX_LABELS, TEXTCAT_MAX_POOL, TEXTCAT_MAX_NGRAM = 128, 1024, 8
 EPI_STORE, EPI_MAXOUT3, EPI_ATOMIC_F32 = 0, 1, 2
 
 
@@ -501,6 +503,43 @@ class B200Ops(TorchOps):
         db = self.colsum(d)
         dX = d @ W
         return loss, d, guesses, dX, dW, db
+
+    # ------------------------------------------------------------------ textcat head
+    def textcat_head(self, X, batch, W, b, W_bow, b_bow, truths, known, *, n_docs=None, use_mean: bool = True,
+                     use_max: bool = False, exclusive: bool = True, no_output_layer: bool = False,
+                     ngram_size: int = 1, grad_out: Optional[Dict[str, torch.Tensor]] = None):
+        """``TorchOps.textcat_head`` in two kernels (textcat_kernels.cu): one CTA per doc for pooling, the
+        bag of n-grams, the output layer, the loss, dX and the W_bow gradient rows; one reduction over docs
+        for dW / db / the loss.  ``n_docs`` may be a device int32 tensor (the engine's packed buffer), so
+        nothing here reads the host.  Gradients accumulate straight into ``grad_out`` (fp32 views of the
+        flat bucket) when given."""
+        weights = [t for t in (W, b, W_bow, b_bow) if t is not None]
+        self._gate_now(*weights)
+        dev = truths.device
+        nL = int(truths.shape[1])
+        go = {k: v for k, v in (grad_out or {}).items()
+              if v is not None and v.dtype == torch.float32 and v.is_contiguous()}
+        grads: Dict[str, torch.Tensor] = {}
+        for name, p in (("W", W), ("b", b), ("W_bow", W_bow), ("b_bow", b_bow)):
+            if p is not None:
+                grads[name] = go[name].view(p.shape) if name in go else torch.zeros(p.shape, dtype=torch.float32,
+                                                                                     device=dev)
+        n_dev, n_host = None, int(batch.doc_lens.numel())
+        if isinstance(n_docs, torch.Tensor):
+            n_dev = n_docs.reshape(-1)[:1]
+        elif n_docs is not None:
+            n_host = int(n_docs)
+        act = 2 if no_output_layer else (0 if exclusive else 1)
+        Xc = X.contiguous() if X is not None else None
+        loss, scores, dX, _pooled, _dl = self.k.textcat_head(
+            Xc, _mask1d(batch.mask).to(torch.float32).contiguous(), batch.attrs.contiguous(), batch.doc_starts,
+            batch.doc_lens, n_dev, n_host, W.contiguous() if W is not None else None,
+            b.contiguous() if b is not None else None, W_bow.contiguous() if W_bow is not None else None,
+            b_bow.contiguous() if b_bow is not None else None, truths.contiguous(), known.contiguous(),
+            grads.get("W"), grads.get("b"), grads.get("W_bow"), grads.get("b_bow"), nL, bool(use_mean),
+            bool(use_max), act, int(ngram_size))
+        self.launches += 2
+        return loss, scores, (dX if X is not None else None), grads
 
     # ------------------------------------------------------------------ K7
     def transition_steps(self, system, Yf, params, batch, gold, is_train):

@@ -360,6 +360,86 @@ void transition_scatter(const Tensor& d_hid, const Tensor& which, const Tensor& 
                                  (int)d_hid.size(0), (int)nF, (int)d_hid.size(1), (int)nP, cur_stream());
 }
 
+// Textcat head: {loss (scalar), scores (B, nL) fp32, dX (Tp, w) bf16 or empty, pooled, d_logits}.  Parameter
+// gradients are ACCUMULATED into gW / gb / gW_bow / gb_bow (fp32; may be views of the flat gradient bucket).
+int weight_is_f32(const c10::optional<Tensor>& t, const char* name) {
+  if (!t.has_value() || !t->defined()) return 0;
+  TORCH_CHECK(t->is_cuda() && t->is_contiguous(), name, " must be a contiguous CUDA tensor");
+  TORCH_CHECK(t->scalar_type() == at::kFloat || t->scalar_type() == at::kBFloat16, name, " must be fp32 or bf16");
+  return t->scalar_type() == at::kFloat ? 1 : 0;
+}
+float* grad_ptr(const c10::optional<Tensor>& t, int64_t numel, const char* name) {
+  if (!t.has_value() || !t->defined()) return nullptr;
+  TORCH_CHECK(t->is_cuda() && t->is_contiguous() && t->scalar_type() == at::kFloat && t->numel() == numel,
+              name, " must be a contiguous fp32 CUDA tensor of ", numel, " elements");
+  return t->data_ptr<float>();
+}
+
+std::vector<Tensor> textcat_head(const c10::optional<Tensor>& X, const Tensor& mask, const Tensor& attrs,
+                                 const Tensor& doc_starts, const Tensor& doc_lens, const c10::optional<Tensor>& n_docs_dev,
+                                 int64_t n_docs, const c10::optional<Tensor>& W, const c10::optional<Tensor>& b,
+                                 const c10::optional<Tensor>& W_bow, const c10::optional<Tensor>& b_bow,
+                                 const Tensor& truths, const Tensor& known, const c10::optional<Tensor>& gW,
+                                 const c10::optional<Tensor>& gb, const c10::optional<Tensor>& gW_bow,
+                                 const c10::optional<Tensor>& gb_bow, int64_t n_labels, bool use_mean, bool use_max,
+                                 int64_t act, int64_t ngram) {
+  SRB_CHECK_CUDA(mask); SRB_CHECK_CUDA(attrs); SRB_CHECK_CUDA(doc_starts); SRB_CHECK_CUDA(doc_lens);
+  SRB_CHECK_CUDA(truths); SRB_CHECK_CUDA(known);
+  TORCH_CHECK(mask.scalar_type() == at::kFloat && attrs.scalar_type() == at::kLong && attrs.dim() == 2 &&
+              doc_starts.scalar_type() == at::kInt && doc_lens.scalar_type() == at::kInt);
+  const int64_t B = doc_lens.numel(), nL = n_labels;
+  TORCH_CHECK(truths.scalar_type() == at::kFloat && known.scalar_type() == at::kFloat &&
+              truths.numel() == B * nL && known.numel() == B * nL, "truths / known must be fp32 (B, n_labels)");
+  const bool has_x = X.has_value() && X->defined();
+  const bool has_w = W.has_value() && W->defined();
+  const bool has_bow = W_bow.has_value() && W_bow->defined();
+  TORCH_CHECK(has_x == has_w, "textcat_head: X and W come together (the pooled branch)");
+  TORCH_CHECK(has_x || has_bow, "textcat_head: nothing to compute");
+  c10::cuda::CUDAGuard guard(attrs.device());
+  srb::TextcatArgs a{};
+  const int64_t Tp = attrs.size(0);
+  const int64_t w = has_x ? X->size(1) : 0;
+  if (has_x) {
+    SRB_CHECK_CUDA(*X); SRB_CHECK_BF16(*X);
+    TORCH_CHECK(X->size(0) == Tp && mask.numel() == Tp);
+  }
+  const int64_t P = (has_x ? (int64_t)use_mean + (int64_t)use_max : 0) * w;
+  a.W_f32 = weight_is_f32(W, "W"); a.b_f32 = weight_is_f32(b, "b");
+  a.W_bow_f32 = weight_is_f32(W_bow, "W_bow"); a.b_bow_f32 = weight_is_f32(b_bow, "b_bow");
+  if (has_w) TORCH_CHECK(W->numel() == nL * P, "W must be (n_labels, n_pool * width)");
+  if (has_bow) TORCH_CHECK(W_bow->dim() == 2 && W_bow->size(1) == nL, "W_bow must be (rows, n_labels)");
+  if (n_docs_dev.has_value() && n_docs_dev->defined()) {
+    TORCH_CHECK(n_docs_dev->is_cuda() && n_docs_dev->scalar_type() == at::kInt && n_docs_dev->numel() >= 1);
+    a.n_docs_dev = n_docs_dev->data_ptr<int32_t>();
+  }
+  auto o = truths.options();
+  Tensor loss = at::empty({}, o);
+  Tensor scores = at::empty({B, nL}, o);
+  Tensor pooled = at::empty({B, P}, o);
+  Tensor d_logits = at::empty({B, nL}, o);
+  Tensor loss_doc = at::empty({B}, o);
+  Tensor dX = has_x ? at::empty({Tp, w}, X->options()) : at::empty({0}, o.dtype(at::kBFloat16));
+  a.X = has_x ? X->data_ptr() : nullptr;
+  a.mask = mask.data_ptr<float>(); a.attrs = attrs.data_ptr<int64_t>();
+  a.doc_starts = doc_starts.data_ptr<int32_t>(); a.doc_lens = doc_lens.data_ptr<int32_t>();
+  a.W = optptr(W); a.b = optptr(b); a.W_bow = optptr(W_bow); a.b_bow = optptr(b_bow);
+  a.truths = truths.data_ptr<float>(); a.known = known.data_ptr<float>();
+  a.scores = scores.data_ptr<float>(); a.pooled = pooled.data_ptr<float>(); a.d_logits = d_logits.data_ptr<float>();
+  a.loss_doc = loss_doc.data_ptr<float>(); a.loss = loss.data_ptr<float>();
+  a.dX = has_x ? dX.data_ptr() : nullptr;
+  a.gW = grad_ptr(gW, nL * P, "gW"); a.gb = grad_ptr(gb, nL, "gb");
+  a.gW_bow = has_bow ? grad_ptr(gW_bow, W_bow->numel(), "gW_bow") : nullptr;
+  a.gb_bow = grad_ptr(gb_bow, nL, "gb_bow");
+  a.bow_rows = has_bow ? W_bow->size(0) : 1;
+  a.n_docs = (int)n_docs; a.B = (int)B; a.Tp = (int)Tp; a.w = (int)w; a.n_attr = (int)attrs.size(1); a.nL = (int)nL;
+  a.use_mean = (has_x && use_mean) ? 1 : 0; a.use_max = (has_x && use_max) ? 1 : 0;
+  a.act = (int)act; a.ngram = has_bow ? (int)ngram : 0;
+  TORCH_CHECK(srb::launch_textcat_head(a, cur_stream()),
+              "textcat_head: outside the kernels' range (labels <= ", srb::kTextcatMaxLabels, ", n_pool * width <= ",
+              srb::kTextcatMaxPool, ", ngram_size <= ", srb::kTextcatMaxNgram, ")");
+  return {loss, scores, dX, pooled, d_logits};
+}
+
 }  // namespace
 
 TORCH_LIBRARY(srb, m) {
@@ -393,6 +473,7 @@ TORCH_LIBRARY(srb, m) {
     srb::launch_bump_i64(t.data_ptr<int64_t>(), by, at::cuda::getCurrentCUDAStream().stream());
   });
   m.def("transition_scatter(Tensor d_hid, Tensor which, Tensor feats, Tensor dYf, Tensor dpad, Tensor db, int nF, int nP) -> ()");
+  m.def("textcat_head(Tensor? X, Tensor mask, Tensor attrs, Tensor doc_starts, Tensor doc_lens, Tensor? n_docs_dev, int n_docs, Tensor? W, Tensor? b, Tensor? W_bow, Tensor? b_bow, Tensor truths, Tensor known, Tensor? gW, Tensor? gb, Tensor? gW_bow, Tensor? gb_bow, int n_labels, bool use_mean, bool use_max, int act, int ngram) -> Tensor[]");
   srb::register_gemm_ops(m);
   srb::register_comm_ops(m);
 }
@@ -414,6 +495,7 @@ TORCH_LIBRARY_IMPL(srb, CUDA, m) {
   m.impl("biluo_steps", biluo_steps);
   m.impl("arc_eager_steps", arc_eager_steps);
   m.impl("transition_scatter", transition_scatter);
+  m.impl("textcat_head", textcat_head);
   srb::register_gemm_impls(m);
   srb::register_comm_impls(m);
 }

@@ -144,6 +144,42 @@ struct ArcArgs {
 };
 bool launch_arc_eager_steps(ArcArgs a, cudaStream_t s);
 int arc_eager_max_doc_len(int nO, int nP, int nA);
+// Textcat head (textcat_kernels.cu): pooling / bag of n-grams -> logits -> softmax | logistic | identity ->
+// d_logits, loss, dX and every parameter gradient, for a whole batch in two launches.
+constexpr int kTextcatMaxLabels = 128;
+constexpr int kTextcatMaxPool = 1024;     // n_pool * width
+constexpr int kTextcatMaxNgram = 8;
+struct TextcatArgs {
+  const void* X;               // bf16 (Tp, w) tok2vec output, or nullptr (bag of words only)
+  const float* mask;           // (Tp) 1.0 on real tokens
+  const int64_t* attrs;        // (Tp, n_attr); column 0 = NORM id (bag of words)
+  const int32_t* doc_starts;   // (B)
+  const int32_t* doc_lens;     // (B)
+  const int32_t* n_docs_dev;   // real doc count on the device, or nullptr: n_docs
+  const void* W;               // (nL, P) output layer or nullptr; P = (use_mean + use_max) * w
+  const void* b;               // (nL) or nullptr
+  const void* W_bow;           // (bow_rows, nL) or nullptr
+  const void* b_bow;           // (nL) or nullptr
+  const float* truths;         // (B, nL)
+  const float* known;          // (B, nL)
+  float* scores;               // (B, nL)
+  float* pooled;               // (B, P) scratch
+  float* d_logits;             // (B, nL) scratch
+  float* loss_doc;             // (B) scratch
+  float* loss;                 // scalar, written
+  void* dX;                    // bf16 (Tp, w) or nullptr
+  float* gW;                   // fp32 gradient accumulators (+=), or nullptr
+  float* gb;
+  float* gW_bow;
+  float* gb_bow;
+  int64_t bow_rows;
+  int n_docs, B, Tp, w, n_attr, nL, use_mean, use_max;
+  int act;                     // 0 softmax, 1 logistic, 2 none (no_output_layer)
+  int ngram;
+  int W_f32, b_f32, W_bow_f32, b_bow_f32;   // weight dtypes: 1 = fp32, 0 = bf16
+};
+// false: shape outside the kernels' range (labels, n_pool * width, ngram_size)
+bool launch_textcat_head(const TextcatArgs& a, cudaStream_t s);
 extern int g_pdl;                                      // launch.h
 // words [0, n_zero) <- 0, [n_zero, n_zero + n_ones) <- 0xFFFFFFFF; both counts multiples of 4, p 16-byte aligned
 void launch_bump_i64(int64_t* p, int64_t by, cudaStream_t s);

@@ -338,6 +338,111 @@ class TorchOps:
         dX = d @ W.to(torch.float32)
         return loss, d, guesses, dX, dW, db
 
+    # ------------------------------------------------------------------ textcat head
+    def textcat_head(self, X, batch, W, b, W_bow, b_bow, truths, known, *, n_docs=None, use_mean: bool = True,
+                     use_max: bool = False, exclusive: bool = True, no_output_layer: bool = False,
+                     ngram_size: int = 1, grad_out: Optional[Dict[str, torch.Tensor]] = None):
+        """Forward + loss + backward of a textcat head over the docs of ``batch`` (device ``doc_starts`` /
+        ``doc_lens``; slots ``>= n_docs`` are unused).  The math of ``models/textcat.py``:
+
+        pooled = [mean | max over the doc's rows of X]; logits = pooled W^T + b (if ``W``)
+                 + sum over the doc's hashed n-grams f of W_bow[f] + b_bow (if ``W_bow``);
+        scores = softmax (exclusive) | logistic | identity (``no_output_layer``);
+        diff = (scores - truths) * known; loss = mean(diff^2) over (n_docs, n_labels);
+        d_logits = diff / n_docs; dX: mean -> d / len, max -> d * [x == max] / n_ties.
+
+        ``n_docs``: int or a 1-element int tensor (None: every slot is a doc).  Gradients are accumulated
+        into ``grad_out[name]`` when given (names ``W``, ``b``, ``W_bow``, ``b_bow``), else fresh tensors.
+        Returns ``(loss, scores, dX, grads)``; ``dX`` is None without ``X``."""
+        dev = truths.device
+        lens = batch.doc_lens.to(device=dev, dtype=torch.int64)
+        starts = batch.doc_starts.to(device=dev, dtype=torch.int64)
+        B = int(lens.numel())
+        n = B if n_docs is None else int(torch.as_tensor(n_docs).reshape(-1)[0])
+        valid = (torch.arange(B, device=dev) < n)
+        lens = torch.where(valid, lens, torch.zeros_like(lens))
+        seg = torch.repeat_interleave(torch.arange(B, device=dev), lens)
+        rows = starts[seg] + (torch.arange(int(lens.sum()), device=dev) - (torch.cumsum(lens, 0) - lens)[seg])
+        nL = int(truths.shape[1])
+        logits = torch.zeros((B, nL), dtype=torch.float32, device=dev)
+        ctx = {}
+        if X is not None:
+            width = X.shape[1]
+            Xt = X.index_select(0, rows).to(torch.float32)
+            inv = 1.0 / lens.clamp(min=1).to(torch.float32).unsqueeze(1)
+            parts = []
+            if use_mean:
+                parts.append(torch.zeros((B, width), dtype=torch.float32, device=dev).index_add_(0, seg, Xt) * inv)
+            if use_max:
+                mx = torch.full((B, width), float("-inf"), dtype=torch.float32, device=dev)
+                mx = mx.scatter_reduce(0, seg.unsqueeze(1).expand(-1, width), Xt, reduce="amax", include_self=True)
+                mx = torch.where(torch.isinf(mx), torch.zeros_like(mx), mx)
+                ctx["argmax"] = (Xt == mx[seg])
+                parts.append(mx)
+            pooled = torch.cat(parts, dim=1)
+            logits = logits + pooled @ W.to(torch.float32).t() + b.to(torch.float32)
+        f = d = None
+        if W_bow is not None:
+            f, d = self._ngram_features(batch.attrs[:, 0].to(dev).index_select(0, rows), seg, ngram_size,
+                                        int(W_bow.shape[0]))
+            logits = logits.index_add(0, d, W_bow.to(torch.float32)[f]) + b_bow.to(torch.float32)
+        if no_output_layer:
+            scores = logits
+        else:
+            scores = torch.softmax(logits, dim=1) if exclusive else torch.sigmoid(logits)
+        scores = scores * valid.unsqueeze(1)
+        diff = (scores - truths.to(torch.float32)) * known.to(torch.float32) * valid.unsqueeze(1)
+        loss = (diff * diff).sum() / (max(n, 1) * nL)
+        d_logits = diff / max(n, 1)
+        go = grad_out or {}
+
+        def acc(name, value):
+            buf = go.get(name)
+            if buf is None:
+                return value
+            buf.view(value.shape).add_(value.to(buf.dtype))
+            return buf
+
+        grads: Dict[str, torch.Tensor] = {}
+        dX = None
+        if W_bow is not None:
+            grads["W_bow"] = acc("W_bow", torch.zeros((W_bow.shape[0], nL), dtype=torch.float32, device=dev)
+                                 .index_add_(0, f, d_logits[d]))
+            grads["b_bow"] = acc("b_bow", d_logits.sum(0))
+        if X is not None:
+            grads["W"] = acc("W", d_logits.t() @ pooled)
+            grads["b"] = acc("b", d_logits.sum(0))
+            d_pooled = d_logits @ W.to(torch.float32)
+            dXt = torch.zeros_like(Xt)
+            off = 0
+            if use_mean:
+                dXt += (d_pooled[:, off:off + width] * inv)[seg]
+                off += width
+            if use_max:
+                hit = ctx["argmax"].to(torch.float32)
+                hit = hit / hit.new_zeros((B, width)).index_add_(0, seg, hit).clamp(min=1.0)[seg]
+                dXt += d_pooled[:, off:off + width][seg] * hit
+            dX = torch.zeros(X.shape, dtype=torch.float32, device=dev)
+            dX.index_copy_(0, rows, dXt)
+            dX = dX.to(X.dtype)
+        return loss, scores, dX, grads
+
+    @staticmethod
+    def _ngram_features(ids: torch.Tensor, seg: torch.Tensor, ngram_size: int, length: int):
+        """``(feature index, doc index)`` of every n-gram (n = 1..ngram_size) of the token-order NORM ids
+        ``ids`` (doc ``seg``): the hash of ``models/textcat.py::_ngram_features``."""
+        feats, docs = [ids], [seg]
+        key = ids
+        for n in range(2, max(1, int(ngram_size)) + 1):
+            if ids.numel() < n:
+                break
+            key = key[:-1] * 1000003 + ids[n - 1:]
+            same = seg[: key.numel()] == seg[n - 1:]
+            feats.append(key[same])
+            docs.append(seg[: key.numel()][same])
+        f = torch.cat(feats)
+        return (f ^ (f >> 31)).remainder(length), torch.cat(docs)
+
     # ------------------------------------------------------------------ K8 Adam (thinc semantics)
     def adam_step(
         self,

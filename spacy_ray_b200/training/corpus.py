@@ -10,7 +10,9 @@ test relies on (``spacy_ray/tests/test_worker.py:26-29``).
 
 ``spacy_ray_b200.SyntheticCorpus.v1`` generates a seeded, *learnable* synthetic
 corpus (there is no network for real data): Zipfian vocabulary, per-type tags,
-capitalised multi-word entities, projective dependency trees.
+capitalised multi-word entities, projective dependency trees, and document
+categories (``textcat``: one of two exclusive classes; ``textcat_multilabel``: two
+independent ones) that follow from which marker words a doc contains.
 """
 from __future__ import annotations
 
@@ -96,6 +98,18 @@ ENT_LABELS = ["PERSON", "ORG", "GPE", "LOC", "PRODUCT", "EVENT", "DATE", "TIME",
               "FAC", "NORP", "LAW", "LANGUAGE", "WORK_OF_ART", "QUANTITY", "ORDINAL", "CARDINAL"]
 DEP_LABELS = ["nsubj", "obj", "det", "amod", "advmod", "case", "nmod", "obl", "cc", "conj", "aux",
               "mark", "compound", "punct", "nummod", "appos"]
+# document categories: a doc "has" a marker when it contains that vocabulary entry.  Entries 2 and 3 of the
+# Zipfian vocabulary occur in roughly half / a third of 24-token docs.
+CAT_MARKERS = (2, 3)
+
+
+def doc_cats(ids: np.ndarray, multilabel: bool) -> Dict[str, float]:
+    """The categories of a doc with vocabulary ids ``ids``: a function of its content alone (no random
+    draw, so adding a textcat task leaves every other annotation of the corpus unchanged)."""
+    has = [bool(np.any(ids == m)) for m in CAT_MARKERS]
+    if multilabel:
+        return {"MARK_A": float(has[0]), "MARK_B": float(has[1])}
+    return {"MARKED": float(has[0]), "PLAIN": float(not has[0])}
 
 
 def _make_word(i: int, rng: np.random.Generator) -> str:
@@ -120,6 +134,8 @@ class SyntheticCorpus:
         self.n_dep_labels = min(int(n_dep_labels), len(DEP_LABELS))
         self.ent_rate, self.noise = float(ent_rate), float(noise)
         self.tasks = tuple(tasks)
+        if "textcat" in self.tasks and "textcat_multilabel" in self.tasks:
+            raise ValueError("SyntheticCorpus: choose one of the tasks 'textcat' / 'textcat_multilabel'")
         self._docs: Optional[List[Doc]] = None
         self._vocab: Optional[Dict[str, Any]] = None
 
@@ -218,6 +234,8 @@ class SyntheticCorpus:
                 heads=heads, deps=deps,
                 attrs=np.ascontiguousarray(attrs_all[ids]),
             )
+            if "textcat" in self.tasks or "textcat_multilabel" in self.tasks:
+                doc.cats = doc_cats(ids, "textcat_multilabel" in self.tasks)
             docs.append(doc)
         self._docs = docs
         return docs

@@ -372,7 +372,7 @@ class Worker:
     def _maybe_install_trainer(self) -> None:
         """On the B200 backend with the fused comm, serve ``nlp.update`` from the
         device-resident engine when the pipeline is one it supports (any mix of tok2vec /
-        tagger / ner / parser components whose heads fit the device kernels).
+        tagger / ner / parser / textcat components whose heads fit the device kernels).
         ``SRB_FAST_PATH=0`` keeps the generic per-op path."""
         ops = get_current_ops()
         if os.environ.get("SRB_FAST_PATH", "1") == "0" or not getattr(ops, "fused", False):
